@@ -12,6 +12,9 @@
 Prints ONE JSON line (see README/DESIGN.md for the field contract).  A train "step" is one full
 train step (forward, losses, backward, grad all-reduce, clip+Adam, weight repack) on one synthetic
 batch of `batch_size` rays (global; sharded B/N per GPU, as train.py:52-53).
+  --dump-outputs DIR   after the timed steps, write what the last timed step returned to its caller as
+                       DIR/<name>.npy (see dump_outputs): the inputs are seeded, so two builds run with the
+                       same arguments can be compared output for output.
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over
 ranks; the activations written per step (>10 GB) exceed the 126 MB L2, so no flush is needed.
 """
@@ -262,6 +265,69 @@ def roofline_block(canon_flops, gemm_ms, gemm_flops, n_gemm, step_ms, clocks, tr
           'whole_step_tflops': whole, 'whole_step_frac': whole / peak if peak else None}
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def sample_positions(size, kept):
+  """Flat (C-order) indices, ascending, of the `kept` elements that dump_outputs writes of an array of `size`."""
+  return np.sort(np.random.default_rng(0).choice(size, kept, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes `arrays` (name -> tensor or ndarray) as <out_dir>/<name>.npy, float64 kept, everything else as
+  float32, DUMP_BYTES in all at most.  The budget is split evenly over the arrays, smallest first; an array
+  larger than its share is written flattened, only its elements at sample_positions(size, kept): the same
+  positions on every run.  <out_dir>/dump.json gives each array's original shape and, when sampled, `kept`."""
+  import torch
+  host = {}
+  for name, v in arrays.items():
+    if isinstance(v, torch.Tensor):
+      v = v.detach().cpu()
+      v = (v if v.dtype == torch.float64 else v.float()).numpy()
+    v = np.asarray(v)
+    host[name] = v if v.dtype == np.float64 else v.astype(np.float32)
+  names = sorted(host, key=lambda k: (host[k].nbytes, k))
+  left = DUMP_BYTES - 256 * len(names) - 65536    # room for the .npy headers and dump.json
+  share = None                                    # set by the first array over its share: all later ones are too
+  index = {}
+  os.makedirs(out_dir, exist_ok=True)
+  for i, name in enumerate(names):
+    v = host[name]
+    index[name] = {'shape': list(v.shape), 'kept': None}
+    if share is None and v.nbytes > left // (len(names) - i):
+      share = left // (len(names) - i)
+    if share is not None:
+      index[name]['kept'] = share // v.itemsize
+      v = v.reshape(-1)[sample_positions(v.size, share // v.itemsize)]
+    left -= v.nbytes
+    np.save(os.path.join(out_dir, name + '.npy'), v)
+  with open(os.path.join(out_dir, 'dump.json'), 'w') as f:
+    json.dump({'arrays': dict(sorted(index.items())),
+               'sampled': 'an array with `kept` set holds only the flattened elements at '
+                          'bench.sample_positions(prod(shape), kept)'}, f, indent=1)
+
+
+def train_outputs(params, stats):
+  """What a train step hands back: the updated state (flat fp32 parameters and Adam moments) and the
+  step's loss statistics."""
+  stats.materialize()
+  out = {'params': params.flat, 'adam_mu': params.mu, 'adam_nu': params.nu, 'mses': stats['mses'],
+         'psnrs': stats['psnrs'], 'loss': np.float64(stats['loss'])}
+  out.update({'loss_' + k: np.float64(v) for k, v in stats['losses'].items()})
+  return out
+
+
+def render_outputs(rendering):
+  """What render_image hands back: the [H, W, ...] image buffers and the per-level ray_* bundles."""
+  out = {}
+  for k, v in rendering.items():
+    if k.startswith('ray_'):
+      out.update({f'{k}_{i}': lv for i, lv in enumerate(v)})
+    else:
+      out[k] = v
+  return out
+
+
 def run_ours(args):
   import torch
   import torch.distributed as dist
@@ -332,7 +398,7 @@ def run_ours(args):
     nonlocal state
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    loss_host = None
+    loss_host = stats = None
     t0 = time.time()
     e0.record()
     for i in range(n):
@@ -343,18 +409,21 @@ def run_ours(args):
     e1.record()
     barrier()
     t1 = time.time()
-    return max_over_ranks(e0.elapsed_time(e1)), loss_host, (t0, t1)
+    return max_over_ranks(e0.elapsed_time(e1)), loss_host, (t0, t1), stats
 
   timed(args.warmup, False)
   ops.LAUNCHES = 0
-  ms, _, win = timed(args.steps, False)
+  ms, _, win, stats = timed(args.steps, False)
   sampler.window(*win)
+  if args.dump_outputs and rank == 0:
+    # before the end-to-end loop below: it keeps training the same state in place
+    dump_outputs(args.dump_outputs, train_outputs(state.params, stats))
   launches_total = ops.LAUNCHES                 # our kernels launched inside the timed region (all K steps)
   launches = launches_total // max(1, args.steps)
   # stop the poller before the end-to-end loop: nvidia-smi queries contend with the driver calls of a loop
   # that synchronises every step (D2H read of the losses)
   clocks = sampler.stop() if rank == 0 else {}
-  ms_e2e, loss_host, _ = timed(args.steps, True)
+  ms_e2e, loss_host, _, _ = timed(args.steps, True)
 
   # dominant kernel (tcgen05 GEMM, all three modes): CUDA events around every launch of one
   # extra step; achieved = canonical train FLOPs of the step / time spent inside the GEMMs
@@ -442,6 +511,8 @@ def run_render(args, wl, bundle, fwd_flop_ray, world, rank, dev, sampler, barrie
   ops.LAUNCHES = 0
   ms, _, out, win = timed(args.steps, False)
   sampler.window(*win)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, render_outputs(out))
   launches_total = ops.LAUNCHES
   clocks = sampler.stop() if rank == 0 else {}
   ms_e2e, img, _, _ = timed(args.steps, True)
@@ -581,7 +652,11 @@ def main():
   ap.add_argument('--cpu_rays', type=int, default=0, help='rays per CPU-arm step (default: the workload\'s)')
   ap.add_argument('--no_cpu_baseline', action='store_true')
   ap.add_argument('--no_graph', action='store_true', help='launch every kernel from Python (no CUDA graphs)')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write what the last timed step returned as DIR/<name>.npy (float32/float64, <= 64 MB in all)')
   args = ap.parse_args()
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs applies to --impl ours')
   if args.impl == 'reference':
     # exactly K timed steps; each step is a bounded ray sample of the workload, shrunk for large K so
     # that the whole run stays within a few minutes of CPU time (1024 rays of 360.gin ~ 3 s per step)

@@ -57,26 +57,37 @@ def test_product_never_imports_oracle():
 
 
 def test_gin_subset_binds_reference_configs():
+  import json
   from multinerf_b200 import configs
   b = configs.bundle_360()
   assert b.config.near == 0.2 and b.config.far == 1e6 and b.model.raydist_fn == 'reciprocal'
   assert b.model.opaque_background and b.nerf_mlp.net_width == 1024 and b.prop_mlp.warp_fn == 'contract'
   assert b.prop_mlp.disable_rgb and b.model.num_levels == 3          # defaults stay
-  ref = '/root/reference/configs'
-  if os.path.isdir(ref):      # build container only: the shipped files must parse unmodified
-    for f in sorted(os.listdir(ref)):
-      if f.endswith('.gin'):
-        configs.load_config([os.path.join(ref, f)], search_paths=[ref, '/root/reference'])
-    r = configs.load_config([os.path.join(ref, 'blender_refnerf.gin')])
-    assert r.nerf_mlp.use_reflections and r.nerf_mlp.deg_view == 5 and r.model.single_mlp
-    assert r.config.orientation_loss_target == 'normals_pred' and r.model.resample_padding == 0.01
-    raw = configs.load_config([os.path.join(ref, 'llff_raw.gin')])
-    assert raw.nerf_mlp.rgb_activation == 'safe_exp' and raw.nerf_mlp.rgb_bias == -5.0
-    assert raw.config.data_loss_type == 'rawnerf' and raw.model.ray_shape == 'cylinder'
-    same = configs.load_config([os.path.join(ref, '360.gin')])
-    assert same == configs.bundle_360()
-    assert configs.load_config([os.path.join(ref, 'blender_256.gin')]) == configs.bundle_blender_256()
-    assert r == configs.bundle_blender_refnerf() and raw == configs.bundle_llff_raw()
+  # the reference's configs/*.gin, byte for byte, and the bindings each one makes (make_golden_configs.py)
+  ref = os.path.join(ROOT, 'tests', 'golden', 'configs')
+  with open(os.path.join(ROOT, 'tests', 'golden', 'configs.json')) as fh:
+    recorded = json.load(fh)
+  assert sorted(f for f in os.listdir(ref) if f.endswith('.gin')) == sorted(recorded) and len(recorded) == 13
+  fields = {'Config': 'config', 'Model': 'model', 'NerfMLP': 'nerf_mlp', 'PropMLP': 'prop_mlp'}
+  for f, cfg in sorted(recorded.items()):      # the shipped files parse unmodified, and every binding we know lands
+    got = configs.load_config([os.path.join(ref, f)], search_paths=[ref])
+    for sel, v in cfg['bindings']:
+      cls, attr = sel.rsplit('.', 1)
+      target = getattr(got, fields[cls])
+      if hasattr(target, attr):
+        assert getattr(target, attr) == (v['ref'].split('.')[-1] if isinstance(v, dict) else v), (f, sel)
+  r = configs.load_config([os.path.join(ref, 'blender_refnerf.gin')])
+  assert r.nerf_mlp.use_reflections and r.nerf_mlp.deg_view == 5 and r.model.single_mlp
+  assert r.config.orientation_loss_target == 'normals_pred' and r.model.resample_padding == 0.01
+  raw = configs.load_config([os.path.join(ref, 'llff_raw.gin')])
+  assert raw.nerf_mlp.rgb_activation == 'safe_exp' and raw.nerf_mlp.rgb_bias == -5.0
+  assert raw.config.data_loss_type == 'rawnerf' and raw.model.ray_shape == 'cylinder'
+  raw_test = configs.load_config([os.path.join(ref, 'llff_raw_test.gin')])      # include + override
+  assert raw_test.config.factor == 0 and raw_test.config.data_loss_type == 'rawnerf'
+  same = configs.load_config([os.path.join(ref, '360.gin')])
+  assert same == configs.bundle_360()
+  assert configs.load_config([os.path.join(ref, 'blender_256.gin')]) == configs.bundle_blender_256()
+  assert r == configs.bundle_blender_refnerf() and raw == configs.bundle_llff_raw()
   b2 = configs.load_config(gin_bindings=['Config.batch_size = 4096', "Model.ray_shape = 'cylinder'",
                                          'NerfMLP.net_activation = @jax.nn.relu', 'Unknown.thing = 3'])
   assert b2.config.batch_size == 4096 and b2.model.ray_shape == 'cylinder' and b2.nerf_mlp.net_activation == 'relu'
@@ -278,6 +289,33 @@ def test_camera_host_helpers():
   assert px.exposure_idx is None and px.exposure_values is None
   with pytest.raises(lib_error()):
     camera_utils.pixels_to_rays(x, y, p, np.eye(4)[:3], device='cpu')      # no CPU path
+
+
+def test_bench_dump_outputs_budget_and_sampling(tmp_path):
+  """bench.py --dump-outputs: float32 / float64 .npy files, DUMP_BYTES in all at most, small arrays whole,
+  the large ones sampled at the same positions on every run."""
+  sys.path.insert(0, ROOT)
+  import bench
+  arrays = {'params': torch.arange(10**7, dtype=torch.float32), 'adam_mu': -torch.arange(10**7, dtype=torch.float32),
+            'mses': torch.ones(3, dtype=torch.bfloat16), 'loss': np.float64(0.25)}
+  for d in ('a', 'b'):
+    bench.dump_outputs(str(tmp_path / d), arrays)
+  a = {p.stem: np.load(p) for p in (tmp_path / 'a').glob('*.npy')}
+  b = {p.stem: np.load(p) for p in (tmp_path / 'b').glob('*.npy')}
+  assert sum(p.stat().st_size for p in (tmp_path / 'a').iterdir()) <= bench.DUMP_BYTES
+  assert a['loss'].dtype == np.float64 and float(a['loss']) == 0.25
+  assert a['mses'].dtype == np.float32 and a['mses'].tolist() == [1.0] * 3
+  assert a['params'].dtype == np.float32 and 0 < a['params'].size < 10**7
+  assert np.all(np.diff(a['params']) > 0)                    # positions in index order, no repeats
+  np.testing.assert_array_equal(a['adam_mu'], -a['params'])  # same positions for same-size arrays
+  for k in a:
+    np.testing.assert_array_equal(a[k], b[k])
+  import json
+  index = json.loads((tmp_path / 'a' / 'dump.json').read_text())['arrays']
+  assert index['mses'] == {'shape': [3], 'kept': None} and index['loss'] == {'shape': [], 'kept': None}
+  assert index['params']['shape'] == [10**7] and index['params']['kept'] == a['params'].size
+  # the sample is traceable: element j of params.npy is params[sample_positions(size, kept)[j]]
+  np.testing.assert_array_equal(a['params'], bench.sample_positions(10**7, index['params']['kept']))
 
 
 def lib_error():
