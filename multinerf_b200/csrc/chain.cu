@@ -156,9 +156,6 @@ mlp_chain_kernel(const __grid_constant__ ChainMaps maps, const ChainParams p) {
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
-  // programmatic dependent launch (see tc_common.cuh): persistent grid, no global access above this line
-  pdl_launch_dependents();
-  pdl_wait();
 
   if (warp == 0) {
     // ===================== TMA producer (both CTAs) =====================
@@ -535,12 +532,10 @@ extern "C" int mnrf_mlp_chain(const mnrf_chain_desc* d, mnrf_stream stream_) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * pairs); cfg.blockDim = dim3(CH_THREADS);
   cfg.dynamicSmemBytes = CH_SMEM; cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
   if (d->mode == MNRF_CHAIN_FWD) {
     static bool set0 = false;
     auto kern = mlp_chain_kernel<0>;

@@ -43,9 +43,12 @@ constexpr int A_STAGE_BYTES = BLOCK_M * BLOCK_K * 2;        // 16 KiB
 constexpr int B_STAGE_BYTES = MAX_BLOCK_N * BLOCK_K * 2;    // 32 KiB
 constexpr int NUM_EPI_WARPS = 8;
 constexpr int OUT_STAGE_BYTES = NUM_EPI_WARPS * 32 * 128;    // one 32-row x 128-byte slab per epilogue warp
-// (operand ring depth, output staging depth): the pair must fit 227 KB of shared memory
-constexpr int smem_bytes(int ctas, int stages, int out_stages) {
-  return stages * (A_STAGE_BYTES + B_STAGE_BYTES / ctas) + out_stages * OUT_STAGE_BYTES + 1024 /*align*/ + 256;
+// Operand ring depth: a CTA of a pair stages half of each B tile, so its ring holds 6 stages where a single CTA's
+// holds 4.  A K = 1024 tile spends 8k cycles in the main loop, so the deepest ring that fits next to one output
+// staging slab per epilogue warp wins (fewer stages with 2 or 3 slabs measured no faster even on K = 256 tiles).
+constexpr int num_stages(int ctas) { return ctas == 2 ? 6 : 4; }
+constexpr int smem_bytes(int ctas) {
+  return num_stages(ctas) * (A_STAGE_BYTES + B_STAGE_BYTES / ctas) + OUT_STAGE_BYTES + 1024 /*align*/ + 256;
 }
 
 constexpr int NUM_THREADS = 128 + NUM_EPI_WARPS * 32;
@@ -77,17 +80,18 @@ struct GemmParams {
   void* out;
 };
 
-template <int MODE, int CTAS, int NUM_STAGES, int OUT_STAGES>
+template <int MODE, int CTAS>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_c, const GemmParams p) {
+  constexpr int NUM_STAGES = num_stages(CTAS);
   constexpr int B_STAGE = B_STAGE_BYTES / CTAS;    // each CTA of a pair stages half of the B tile
   extern __shared__ uint8_t smem_dyn[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_dyn) + 1023) & ~uintptr_t(1023));
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + NUM_STAGES * A_STAGE_BYTES;
   uint8_t* smem_out = smem + NUM_STAGES * (A_STAGE_BYTES + B_STAGE);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_out + OUT_STAGES * OUT_STAGE_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_out + OUT_STAGE_BYTES);
   uint64_t* full_bar = bars;                       // [NUM_STAGES]  (CTAS=2: the leader's are used)
   uint64_t* empty_bar = bars + NUM_STAGES;         // [NUM_STAGES]
   uint64_t* tfull_bar = bars + 2 * NUM_STAGES;     // [NUM_ACC]
@@ -125,10 +129,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
   if (CTAS == 1) __syncthreads(); else cluster_sync_all();    // peers must see initialised barriers
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
-  // Programmatic dependent launch: this grid is persistent (every CTA resident from the start), so the next grid may
-  // take each SM the moment this grid's CTA leaves it; nothing above touched global memory, everything below does.
-  pdl_launch_dependents();
-  pdl_wait();
 
   const int b_rows = p.block_n / CTAS;             // B-tile rows this CTA stages
   const uint32_t stage_bytes = A_STAGE_BYTES + (uint32_t)b_rows * BLOCK_K * 2;
@@ -238,7 +238,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     float csacc[4] = {0.f, 0.f, 0.f, 0.f};     // tiles 0, 2, 4, ... of this CTA (all tiles for period 1)
     float csodd[4] = {0.f, 0.f, 0.f, 0.f};     // tiles 1, 3, 5, ... (period 2)
     int cs_ncol0 = -1, cs_ncol1 = -1;
-    uint32_t store_it = 0;
     uint32_t sstage = 0, sphase = 0;        // WGRAD side sums: this warp's position in the operand ring
 
     // per-row inputs of a tile (DGRAD): fetched one tile ahead so their latency hides behind the
@@ -494,11 +493,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
         if (p.use_tma_store) {
           // 64-column groups: two 32-column halves share one 32x128-byte swizzled staging slab
           const int half = ci & 1;
-          uint8_t* slab = smem_out + (ew * OUT_STAGES + (store_it % OUT_STAGES)) * (32 * 128);
+          uint8_t* slab = smem_out + ew * (32 * 128);
           const uint32_t slab_s = smem_u32(slab) + lane * 128;
           if (half == 0) {
             // the bulk store previously issued from this slab must have finished reading it
-            if (lane == 0) tma_store_wait_read<OUT_STAGES - 1>();
+            if (lane == 0) tma_store_wait_read<0>();
             __syncwarp();
           }
 #pragma unroll
@@ -513,7 +512,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
               tma_store_2d(&tmap_c, slab, ncol0 + c0 - 32, m_blk * BLOCK_M + q * 32);
               tma_store_commit();
             }
-            ++store_it;
           }
         } else if (row_ok) {
           uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.out) + row * p.ldc + col);
@@ -606,9 +604,6 @@ int gemm_tc_launch(const mnrf_gemm_desc* d, const mnrf_bf16* a, const mnrf_bf16*
   if (bias) MNRF_CHECK(((uintptr_t)bias % 16) == 0, "mnrf_gemm(tc): bias must be 16-byte aligned");
   if (colv) MNRF_CHECK(((uintptr_t)colv % 16) == 0, "mnrf_gemm(tc): colv must be 16-byte aligned");
   p.use_tma_store = (d->mode != MNRF_GEMM_WGRAD && p.block_n % 64 == 0) ? 1 : 0;
-  static const int cfg_ctas = getenv("MNRF_GEMM_CTAS") ? atoi(getenv("MNRF_GEMM_CTAS")) : 2;
-  static const int cfg_stages = getenv("MNRF_GEMM_STAGES") ? atoi(getenv("MNRF_GEMM_STAGES")) : 0;
-  static const int cfg_smallk = getenv("MNRF_GEMM_SMALLK") ? atoi(getenv("MNRF_GEMM_SMALLK")) : 0;
 #ifdef MNRF_TIMING_KNOBS
   // timing experiments only (results are wrong by construction): compiled in only on request
   static const int cfg_debug = getenv("MNRF_GEMM_DEBUG") ? atoi(getenv("MNRF_GEMM_DEBUG")) : 0;
@@ -618,7 +613,7 @@ int gemm_tc_launch(const mnrf_gemm_desc* d, const mnrf_bf16* a, const mnrf_bf16*
   p.debug = cfg_debug;
   const int sms = mnrf_num_sms();
   // CTA pairs (tcgen05 cta_group::2) whenever the tile grid is made of whole 256 x 256 tiles
-  const int ctas = (cfg_ctas == 2 && p.block_n == MAX_BLOCK_N && d->m % (2 * BLOCK_M) == 0 && sms % 2 == 0) ? 2 : 1;
+  const int ctas = (p.block_n == MAX_BLOCK_N && d->m % (2 * BLOCK_M) == 0 && sms % 2 == 0) ? 2 : 1;
   const int workers = sms / ctas;
   p.num_splits = 1;
   if (d->mode == MNRF_GEMM_WGRAD) {
@@ -659,12 +654,12 @@ int gemm_tc_launch(const mnrf_gemm_desc* d, const mnrf_bf16* a, const mnrf_bf16*
   const int total_tiles = (p.num_m_blocks / ctas) * p.num_n_blocks * p.num_splits;
   const int grid = std::min(total_tiles, workers) * ctas;
   if (grid == 0) return 0;
-#define MNRF_LAUNCH_TC2(MODE_, CTAS_, ST_, OST_)                                                      \
+#define MNRF_LAUNCH_TC(MODE_, CTAS_)                                                                  \
   do {                                                                                                \
     static bool attr_set = false;                                                                     \
-    constexpr int kSmem = smem_bytes(CTAS_, ST_, OST_);                                               \
+    constexpr int kSmem = smem_bytes(CTAS_);                                                          \
     static_assert(kSmem <= 232448, "shared memory budget");                                           \
-    auto kern = gemm_tc_kernel<MODE_, CTAS_, ST_, OST_>;                                              \
+    auto kern = gemm_tc_kernel<MODE_, CTAS_>;                                                         \
     if (!attr_set) {                                                                                  \
       MNRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem));      \
       attr_set = true;                                                                                \
@@ -672,33 +667,21 @@ int gemm_tc_launch(const mnrf_gemm_desc* d, const mnrf_bf16* a, const mnrf_bf16*
     cudaLaunchConfig_t cfg = {};                                                                      \
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(NUM_THREADS);                                       \
     cfg.dynamicSmemBytes = kSmem; cfg.stream = stream;                                                \
-    cudaLaunchAttribute attr[2];                                                                      \
+    cudaLaunchAttribute attr[1];                                                                      \
     attr[0].id = cudaLaunchAttributeClusterDimension;                                                 \
     attr[0].val.clusterDim.x = CTAS_; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;     \
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                  \
-    attr[1].val.programmaticStreamSerializationAllowed = 1;                                           \
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 2 : 1;                                           \
+    cfg.attrs = attr; cfg.numAttrs = 1;                                                               \
     MNRF_CUDA(cudaLaunchKernelEx(&cfg, kern, ta, tb, tc, p));                                         \
   } while (0)
-  // Ring depth vs output staging (CTA pairs): a K = 1024 tile spends 8k cycles in the main loop, so the deepest
-  // operand ring wins and one staging slab per epilogue warp is enough; a short-K tile (K <= 512: the bottleneck /
-  // view-branch input gradients) is paced by its epilogue, where a warp that owns ONE slab stalls on the bulk
-  // store that is still reading it -- those shapes take fewer operand stages and 2 or 3 slabs (MNRF_GEMM_SMALLK).
-  int stages_sel = cfg_stages;
-  if (stages_sel == 0 && d->mode != MNRF_GEMM_WGRAD && p.num_k_blocks <= 8) stages_sel = cfg_smallk;
-#define MNRF_LAUNCH_TC(MODE_)                                                                         \
-  do {                                                                                                \
-    if (ctas == 2) {                                                                                  \
-      if (stages_sel == 5) MNRF_LAUNCH_TC2(MODE_, 2, 5, 2);                                           \
-      else if (stages_sel == 4) MNRF_LAUNCH_TC2(MODE_, 2, 4, 3);                                      \
-      else MNRF_LAUNCH_TC2(MODE_, 2, 6, 1);                                                           \
-    } else {                                                                                          \
-      MNRF_LAUNCH_TC2(MODE_, 1, 4, 1);                                                                \
-    }                                                                                                 \
-  } while (0)
-  if (d->mode == MNRF_GEMM_FWD) MNRF_LAUNCH_TC(MNRF_GEMM_FWD);
-  else if (d->mode == MNRF_GEMM_DGRAD) MNRF_LAUNCH_TC(MNRF_GEMM_DGRAD);
-  else MNRF_LAUNCH_TC(MNRF_GEMM_WGRAD);
+  if (ctas == 2) {
+    if (d->mode == MNRF_GEMM_FWD) MNRF_LAUNCH_TC(MNRF_GEMM_FWD, 2);
+    else if (d->mode == MNRF_GEMM_DGRAD) MNRF_LAUNCH_TC(MNRF_GEMM_DGRAD, 2);
+    else MNRF_LAUNCH_TC(MNRF_GEMM_WGRAD, 2);
+  } else {
+    if (d->mode == MNRF_GEMM_FWD) MNRF_LAUNCH_TC(MNRF_GEMM_FWD, 1);
+    else if (d->mode == MNRF_GEMM_DGRAD) MNRF_LAUNCH_TC(MNRF_GEMM_DGRAD, 1);
+    else MNRF_LAUNCH_TC(MNRF_GEMM_WGRAD, 1);
+  }
   MNRF_LAUNCH_CHECK();
   return 0;
 }

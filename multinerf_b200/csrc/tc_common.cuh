@@ -203,14 +203,6 @@ __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float 
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
-// Programmatic dependent launch (the launch carries cudaLaunchAttributeProgrammaticStreamSerialization when
-// MNRF_PDL=1): `pdl_launch_dependents` lets the NEXT grid of the stream become resident as this grid's CTAs exit
-// (its prologue -- barrier init, TMEM allocation, tensor-map prefetch, cluster sync -- then overlaps this grid's
-// tail); `pdl_wait` blocks until every prerequisite grid has completed and flushed its memory, so it must precede
-// the first access to global memory.  Both are no-ops for a launch without the attribute.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // Shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): 128-byte swizzle, version 1.
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
@@ -235,12 +227,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
                                   CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
                                   CUtensorMapFloatOOBfill);
-
-// MNRF_PDL=1: tensor-core kernels are launched as programmatic dependents of the previous kernel of the stream
-inline bool pdl_enabled() {
-  static const bool on = getenv("MNRF_PDL") != nullptr && atoi(getenv("MNRF_PDL")) != 0;
-  return on;
-}
 
 inline EncodeTiledFn get_encode_fn() {
   static EncodeTiledFn fn = nullptr;

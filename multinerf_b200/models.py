@@ -609,8 +609,7 @@ class Model:
   # ------------------------------------------------------------------ layer-chained 256-wide trunks
   def _use_chain(self, plan, M, impl=0):
     """One persistent launch per trunk (csrc/chain.cu) when every trunk layer is 256 wide."""
-    import os
-    if impl != 0 or os.environ.get('MNRF_CHAIN', '1') == '0':
+    if impl != 0:
       return False
     cfg = plan.cfg
     return (cfg.net_width == 256 and cfg.net_depth <= L.CHAIN_MAX_LAYERS and M >= 512 and

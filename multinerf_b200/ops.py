@@ -149,22 +149,11 @@ def gemm(mode, a, b, out, *, m, n, k, act=L.ACT_NONE, bias=None, rowv=None, colv
   return out
 
 
-import os as _os
-_NO_SIDE_SUMS = _os.environ.get('MNRF_SIDE_SUMS', '1') == '0'
-
-
 def gemm_wgrad(x, dy, out, *, m, n, k, bsum=None, side_w=None, side_aw=None, impl=0):
   """dW[m, n] += x[k, m]^T dy[k, n], plus (optional) bsum[n] += column sums of dy (the layer's bias gradient) and
   side_aw[m] += sum_r side_w[r] x[r, m] (weight gradient of a Dense(1) head on x) -- include/mnrf.h."""
   lib = L.load()
   assert x.stride(-1) == 1 and dy.stride(-1) == 1 and out.stride(-1) == 1
-  if _NO_SIDE_SUMS:        # A/B switch for profiling: the same sums as separate passes over HBM
-    gemm(L.GEMM_WGRAD, x, dy, out, m=m, n=n, k=k, impl=impl)
-    if bsum is not None:
-      colsum(dy, n, bsum)
-    if side_aw is not None:
-      head_bwd(x, x, side_w.view(-1, 1), 1, m, dx=None, dw=side_aw.view(-1, 1), db=None)
-    return out
   d = L.GemmDesc(L.GEMM_WGRAD, L.ACT_NONE, m, n, k, x.stride(0), dy.stride(0), out.stride(0), 0, 0, 0, 0, impl)
   _count()
   ev = None

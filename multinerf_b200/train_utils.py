@@ -70,8 +70,9 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
   on the device from `cameras` first (train_utils.py:266-268; camera type from `dataset.camtype`
   as train_utils.py:234-237).
 
-  use_graph=True captures the step into two CUDA graphs (forward+backward | clip+Adam+repack,
-  with the NCCL all-reduce between them) after one eager warm-up step; per-step scalars
+  use_graph=True captures the step after one eager warm-up step: into ONE CUDA graph on a single GPU
+  (forward + backward + clip/Adam/repack), into TWO when data-parallel (forward + backward | clip +
+  Adam + repack, with the NCCL all-reduce between the replays); per-step scalars
   (annealing exponent, learning rate, Adam bias corrections) and the jitter draws live in device
   buffers that are refreshed before each replay, so train_frac and the step count may advance.
   """
@@ -107,28 +108,6 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
   anneal_dev = dyn[3:4]
   G = {'state': 0, 'fb': None, 'opt': None, 'rays': None, 'target': None, 'jitter': None,
        'noise': None, 'launches': 0}
-  import os
-  # capturing the NCCL all-reduce inside the step graph hangs on this stack (torch 2.11 / NCCL 2.28, measured on
-  # 2 x B200 in round 2): opt-in only
-  GRAPH_NCCL = os.environ.get('MNRF_GRAPH_NCCL', '0') == '1'
-  EARLY_EXCHANGE = os.environ.get('MNRF_EARLY_EXCHANGE', '0') == '1'
-
-  # Backward runs the levels last to first, so a module's gradient is final once the lowest level that
-  # uses it is done: for 360.gin the NerfMLP segment (34.7 of 36 MB) is final after level 2 and its
-  # all-reduce overlaps the two PropMLP backward levels.
-  def early_segments(n_levels):
-    # Opt-in (MNRF_EARLY_EXCHANGE=1).  Measured on 2 and 8 x B200 (round 2): overlapping the NerfMLP all-reduce with
-    # the PropMLP backward is a LOSS here -- the backward kernels are persistent, one CTA (pair) per SM with all of
-    # its shared memory, so they cannot share SMs with NCCL's channel CTAs; every overlapped kernel waits for the
-    # collective on the SMs it needs (8 GPUs: 4.55 ms/step overlapped vs 4.31 ms with the exchange after the backward).
-    if decay_views or not EARLY_EXCHANGE:
-      return {}                      # weight decay touches every gradient after the last level
-    first_use = {}
-    for i in range(n_levels):
-      mname = 'NerfMLP_0' if (mcfg.single_mlp or i == n_levels - 1) else 'PropMLP_0'
-      first_use.setdefault(mname, i)
-    return {i: mname for mname, i in first_use.items() if i > 0}
-
   def fb_begin(rng, rays, target, train_frac, anneal_ptr):
     """Zero the gradients, run the forward pass of every level; returns the context of the backward pass."""
     params = model.params
@@ -171,41 +150,13 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
     model._mlp_backward(st, model.mlps[st.mname], rays=rays, impl=impl, loss_mults=st.loss_mults,
                         stats=ctx['stats'][i])
 
-  def split_level(n_levels, world):
-    """Level after whose backward the first gradient segment is final (None: exchange everything at the end)."""
-    early = early_segments(n_levels) if world > 1 else {}
-    return (max(early), early[max(early)]) if early else (None, None)
-
-  def exchange_early(params, mname):
-    o, cnt = params.offsets[mname]
-    return dist.all_reduce(params.grads_ext[o:o + cnt], op=dist.ReduceOp.SUM, async_op=True), (o, o + cnt)
-
-  def exchange_rest(params, done, pending):
-    """Everything not yet exchanged (contiguous ranges of the flat buffer, statistics tail included)."""
-    pos = 0
-    for lo, hi in sorted(done) + [(params.grads_ext.numel(), params.grads_ext.numel())]:
-      if lo > pos:
-        dist.all_reduce(params.grads_ext[pos:lo], op=dist.ReduceOp.SUM)
-      pos = hi
-    for w in pending:
-      w.wait()
-
-  def fwd_bwd(rng, rays, target, train_frac, anneal_ptr, world=1):
-    """Eager step body: forward, backward last level to first, gradient exchange (world > 1)."""
+  def fwd_bwd(rng, rays, target, train_frac, anneal_ptr):
+    """Forward, backward last level to first, weight decay: the parameter gradients of this rank's shard."""
     ctx = fb_begin(rng, rays, target, train_frac, anneal_ptr)
-    n = len(ctx['states'])
-    split, seg = split_level(n, world)
-    pending, done = [], []
-    for i in range(n - 1, -1, -1):
+    for i in range(len(ctx['states']) - 1, -1, -1):
       fb_level(ctx, i)
-      if i == split:
-        w, rng_ = exchange_early(ctx['params'], seg)
-        pending.append(w)
-        done.append(rng_)
     if decay_views:
       weight_decay()
-    if world > 1:
-      exchange_rest(ctx['params'], done, pending)
 
   def weight_decay():
     # loss += mult * sum(w^2)  ->  grad += 2 mult w ; the loss value goes to stats row 0, slot 6
@@ -309,7 +260,8 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
                              config.lr_delay_steps, config.lr_delay_mult)
     if not use_graph or G['state'] == 0:
       # eager step (also the warm-up that allocates every buffer before a capture)
-      fwd_bwd(draw_randomness(rng, B, sched) if use_graph else rng, rays, target, train_frac, None, world)
+      fwd_bwd(draw_randomness(rng, B, sched) if use_graph else rng, rays, target, train_frac, None)
+      allreduce_flat_(params, world)
       optim(grad_scale, params.step, lr, None)
       G['state'] = 1 if use_graph else 0
       G['B'] = B
@@ -329,38 +281,18 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
       G['target'] = target.clone()
       torch.cuda.synchronize()
       before = ops.LAUNCHES
-      n_lv = len(sched)
-      split, seg = split_level(n_lv, world)
-      G['split'] = None
-      if world > 1 and not GRAPH_NCCL:
-        # NCCL stays outside the graphs (capturing it hung on this stack, round 2): the step is two graphs around
-        # the exchange, or THREE when a gradient segment is final early -- [forward + backward down to the split
-        # level] | async all-reduce of that segment | [remaining backward levels] | all-reduce of the rest |
-        # [clip + Adam + repack] -- so the big NerfMLP exchange overlaps the PropMLP backward
-        G['fb'] = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(G['fb']):
-          ctx = fb_begin(rand, G['rays'], G['target'], train_frac, anneal_dev)
-          for i in range(n_lv - 1, (split if split is not None else 0) - 1, -1):
-            fb_level(ctx, i)
-          if split is None and decay_views:
-            weight_decay()
-        if split is not None:
-          G['split'] = seg
-          G['fb2'] = torch.cuda.CUDAGraph()
-          with torch.cuda.graph(G['fb2'], pool=G['fb'].pool()):
-            for i in range(split - 1, -1, -1):
-              fb_level(ctx, i)
+      G['fb'] = torch.cuda.CUDAGraph()
+      with torch.cuda.graph(G['fb']):
+        fwd_bwd(rand, G['rays'], G['target'], train_frac, anneal_dev)
+        if world == 1:
+          optim(grad_scale, params.step, lr, dyn)
+      G['opt'] = None
+      if world > 1:
+        # NCCL stays outside the graphs (capturing the all-reduce hung on torch 2.11 / NCCL 2.28, 2 x B200):
+        # the all-reduce runs between the replays of the two graphs
         G['opt'] = torch.cuda.CUDAGraph()
         with torch.cuda.graph(G['opt']):
           optim(grad_scale, params.step, lr, dyn)
-      else:
-        # ONE graph for the whole step: forward, backward, (world > 1: the gradient all-reduces, captured on
-        # NCCL's stream as parallel branches), clip + Adam + weight repack
-        G['fb'] = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(G['fb']):
-          fwd_bwd(rand, G['rays'], G['target'], train_frac, anneal_dev, world)
-          optim(grad_scale, params.step, lr, dyn)
-        G['opt'] = None
       G['launches'] = ops.LAUNCHES - before
       G['state'] = 2
     else:
@@ -381,12 +313,7 @@ def create_train_step(model: models.Model, config: configs.Config, impl=0, use_g
         torch._foreach_copy_(dd, ss, non_blocking=True)
     G['fb'].replay()
     if G['opt'] is not None:
-      if G['split'] is not None:
-        w, rng_ = exchange_early(params, G['split'])
-        G['fb2'].replay()
-        exchange_rest(params, [rng_], [w])
-      else:
-        allreduce_flat_(params, world)
+      allreduce_flat_(params, world)
       G['opt'].replay()
     ops.LAUNCHES += G['launches']
     return state, LazyStats(stats_view(params).clone(), n, grad_scale), rng
@@ -453,17 +380,6 @@ def allreduce_flat_(params, world):
   1/world factor is applied downstream (clip_adam grad_scale, LazyStats scale)."""
   if world > 1:
     dist.all_reduce(params.grads_ext, op=dist.ReduceOp.SUM)
-  return 1.0 / world
-
-
-def allreduce_mean_(grads, stats, world):
-  """pmean of gradients and stats (train_utils.py:319-321): SUM all-reduce here, the 1/world
-  factor is applied to the gradient inside clip_adam (grad_scale) and to the stats in place."""
-  if world <= 1:
-    return 1.0
-  dist.all_reduce(grads, op=dist.ReduceOp.SUM)
-  dist.all_reduce(stats, op=dist.ReduceOp.SUM)
-  stats.div_(world)
   return 1.0 / world
 
 

@@ -4,7 +4,6 @@ tcgen05 GEMMs (mnrf_gemm) and a plain fp32 torch product of the same bf16 operan
 Reference being replaced: the Dense + ReLU loop of internal/models.py:441-465 (forward, skip concat at
 :458-459) and its reverse-mode input-gradient chain."""
 import math
-import os
 
 import numpy as np
 import pytest
@@ -164,8 +163,8 @@ def test_chain_rejects_bad_descriptors(ops):
     ops.mlp_chain((d, fl))
 
 
-def test_model_chain_matches_per_layer_path():
-  """The same train step with the chained trunks (default) and with MNRF_CHAIN=0 (per-layer GEMMs).
+def test_model_chain_matches_per_layer_path(monkeypatch):
+  """The same train step with the chained trunks (default) and with the per-layer GEMMs.
   `blender1`: one level of the 8 x 256 NerfMLP (skip connection) -- no resampling between the two paths, so the
   gradients agree to rounding.  `360`: PropMLP chained, and the two paths differ by the summation order of
   the density head (1e-7 relative), which moves the resampled positions of the next level by a few ulps;
@@ -176,9 +175,10 @@ def test_model_chain_matches_per_layer_path():
   lib.require_device()
   for which, tol in (('blender1', 5e-3), ('360', 0.2)):
     grads = []
-    for chain in ('1', '0'):
-      os.environ['MNRF_CHAIN'] = chain
-      try:
+    for chain in (True, False):
+      with monkeypatch.context() as mp:
+        if not chain:
+          mp.setattr(models.Model, '_use_chain', lambda self, plan, M, impl=0: False)
         bundle = configs.bundle_360() if which == '360' else configs.bundle_blender_256()
         if which == 'blender1':
           bundle.model.num_levels = 1
@@ -196,8 +196,6 @@ def test_model_chain_matches_per_layer_path():
         state, stats, _ = step_fn(rand, state, utils.Batch(rays=rays, rgb=target), None, 0.5)
         torch.cuda.synchronize()
         grads.append((model.export_grads_flax(), stats.materialize()['loss']))
-      finally:
-        os.environ.pop('MNRF_CHAIN', None)
     (g1, l1), (g0, l0) = grads
     assert abs(l1 - l0) < (1e-4 if which == 'blender1' else 1e-2) * max(1.0, abs(l0)), (which, l1, l0)
     for mname in g1:

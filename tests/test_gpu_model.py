@@ -7,6 +7,7 @@ oracle/o_models.py `bf16=True`.  Achieved errors are asserted with explicit tole
 """
 import copy
 import math
+import os
 
 import numpy as np
 import pytest
@@ -200,7 +201,7 @@ def test_train_step_vs_oracle(mods, which, impl):
 
 
 def test_cuda_graph_train_step_matches_eager(mods):
-  """The captured two-graph step (forward+backward | clip+Adam+repack) must track the eager step
+  """The captured one-graph step (forward + backward + clip/Adam/repack) must track the eager step
   while train_frac, the learning rate, the Adam bias corrections and the jitter change per step."""
   models, train_utils = mods
   from multinerf_b200 import utils
@@ -233,6 +234,79 @@ def test_cuda_graph_train_step_matches_eager(mods):
   # fp32 atomics make the two runs differ in the last bits only
   rel = float((p0 - p1).norm() / p0.norm())
   assert rel < 2e-3, rel
+
+
+def _data_parallel_worker(rank, world, port, q):
+  """One rank of the world-2 graph-vs-eager check: its own half of the rays, both ranks on cuda:0."""
+  import traceback
+  import torch.distributed as dist
+  try:
+    os.environ['MASTER_ADDR'] = '127.0.0.1'
+    os.environ['MASTER_PORT'] = str(port)
+    dist.init_process_group('gloo', rank=rank, world_size=world)
+    from multinerf_b200 import lib, models, train_utils, utils
+    lib.require_device()
+    torch.cuda.set_device(0)
+    bundle = mini360()
+    # The global-norm clip sums the gradient norm with fp32 atomics, whose order differs between processes; without
+    # it the update is elementwise, so replicas that apply the same all-reduced gradient stay bit-identical.
+    bundle.config.grad_max_norm = 0.0
+    B, steps = 256, 4
+    rays, rng = synth_rays(5, B, 0.2, 1e6)
+    shard = lambda x: x[rank * B:(rank + 1) * B]
+    batches = [(synth_rays(10 + i, world * B, 0.2, 1e6)[0].map(shard),
+                shard(rng.uniform(0, 1, (world * B, 3)).astype(np.float32))) for i in range(steps)]
+    rands = [{'jitter': [torch.tensor(shard(rng.uniform(0, 1, (world * B,)).astype(np.float32))) for _ in range(3)]}
+             for _ in range(steps)]
+    out = {}
+    for use_graph in (False, True):
+      model, variables = models.construct_model(6, rays, bundle)
+      step_fn = train_utils.create_train_step(model, bundle.config, use_graph=use_graph)
+      state = train_utils.TrainState(variables)
+      losses = []
+      for i in range(steps):
+        state, stats, _ = step_fn(rands[i], state, utils.Batch(rays=batches[i][0], rgb=batches[i][1]), None, i / 10.0)
+        losses.append(stats.materialize()['loss'])
+      torch.cuda.synchronize()
+      g = step_fn.graph_info
+      out[use_graph] = (losses, variables.flat.cpu().numpy(), g['state'], g['opt'] is not None)
+    q.put((rank, out, None))
+    dist.destroy_process_group()
+  except Exception:  # pylint: disable=broad-except
+    q.put((rank, None, traceback.format_exc()))
+
+
+def test_cuda_graph_train_step_world_size_2_matches_eager():
+  """Data-parallel step at world size 2 (two processes on one device, gloo all-reduce): the two captured graphs
+  (forward + backward | clip + Adam + repack) with the all-reduce between the replays must track the eager step,
+  and both ranks must end with the same parameters."""
+  import torch.multiprocessing as mp
+  ctx = mp.get_context('spawn')
+  q = ctx.Queue()
+  port = 29900 + os.getpid() % 90
+  procs = [ctx.Process(target=_data_parallel_worker, args=(r, 2, port, q)) for r in range(2)]
+  for p in procs:
+    p.start()
+  res = {}
+  try:
+    for _ in range(2):
+      rank, out, err = q.get(timeout=300)
+      assert err is None, f'rank {rank}:\n{err}'
+      res[rank] = out
+  finally:
+    for p in procs:
+      p.join(60)
+      if p.is_alive():             # a rank that failed leaves its peer waiting in a collective
+        p.terminate()
+  for out in res.values():
+    (l0, p0, _, _), (l1, p1, state, two_graphs) = out[False], out[True]
+    assert state == 2 and two_graphs
+    for a, b in zip(l0, l1):
+      assert abs(a - b) < 2e-3 * max(1.0, abs(a)), (l0, l1)
+    rel = float(np.linalg.norm(p0 - p1) / np.linalg.norm(p0))
+    assert rel < 2e-3, rel
+  for use_graph in (False, True):
+    np.testing.assert_array_equal(res[0][use_graph][1], res[1][use_graph][1])
 
 
 def test_cuda_graph_gradients_track_eager_with_moving_weights(mods):

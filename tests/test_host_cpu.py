@@ -201,9 +201,6 @@ def _gloo_worker(rank, world, port, q):
   dist.init_process_group('gloo', rank=rank, world_size=world)
   sys.path.insert(0, ROOT)
   from multinerf_b200 import train_utils
-  grads = torch.full((10,), float(rank + 1))
-  stats = torch.full((3, 8), float(rank))
-  scale = train_utils.allreduce_mean_(grads, stats, world)
   rend = [{'rgb': torch.full((4, 3), float(rank)), 'acc': torch.arange(4.) + 10 * rank,
            'ray_sdist': torch.full((2, 5), float(rank))}]
   g = train_utils.gather_renderings(rend, world)
@@ -219,8 +216,7 @@ def _gloo_worker(rank, world, port, q):
   prm.stats_tail.fill_(float(rank))
   assert train_utils.allreduce_flat_(prm, world) == 0.5
   assert float(prm.grads.min()) == float(prm.grads.max()) == 3.0 and float(prm.stats_tail.max()) == 1.0
-  q.put((rank, grads.tolist(), stats[0, 0].item(), scale, g[0]['rgb'][:, 0].tolist(), g[0]['acc'].tolist(),
-         g[0]['ray_sdist'][0, 0].item()))
+  q.put((rank, g[0]['rgb'][:, 0].tolist(), g[0]['acc'].tolist(), g[0]['ray_sdist'][0, 0].item()))
   dist.destroy_process_group()
 
 
@@ -235,9 +231,7 @@ def test_world_size_2_collectives_gloo():
   res = sorted(q.get(timeout=60) for _ in range(2))
   for p in procs:
     p.join(30)
-  for rank, grads, st, scale, rgb, acc, rs in res:
-    assert grads == [3.0] * 10 and scale == 0.5           # SUM all-reduce; mean applied via grad_scale
-    assert st == 0.5                                      # stats pmean
+  for rank, rgb, acc, rs in res:
     assert rgb == [0.0] * 4 + [1.0] * 4                   # rank r's rows at [r*n, (r+1)*n)
     assert acc == [0., 1., 2., 3., 10., 11., 12., 13.]
     assert rs == float(rank)                              # ray_* bundles stay local
